@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path
     python bench.py --impl reference --gpus N --steps K --warmup W   # the reference's CPU path (oracle port) on host cores
+    python bench.py --gpus 1 --steps K --warmup W --dump-outputs DIR  # also write the last timed step's outputs to DIR/*.npy
 
 Workload (BASELINE.json configs[1], SURVEY 8d-2): VibeVoice-1.5B, 1 speaker, 64K context = 63,488-token synthetic prompt +
 2,047 generated speech frames (context ends at 65,535 = max_position_embeddings - 1; 273 s of audio per step), 30 diffusion
@@ -35,6 +36,7 @@ import numpy as np
 import torch
 
 AUDIO_S_PER_FRAME = 3200.0 / 24000.0
+DUMP_BYTES = 64 * 10**6          # --dump-outputs: size of everything it writes, at most
 # DRAM traffic of one frame / one LM step from an ncu pass (dram__bytes_read.sum + dram__bytes_write.sum over every kernel of the frame),
 # see profiles/ (filled in by the profiling run of this round; None = not captured for that model)
 TRAFFIC_NOTE = {
@@ -63,7 +65,33 @@ def parse():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-7b", action="store_true", help="skip the VibeVoice-7B sub-configs appended to the 1.5B line")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed step computed as DIR/<name>.npy (float32, %d MB at most in "
+                         "all: a fixed, seeded sample of each array beyond that)" % (DUMP_BYTES // 10**6))
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs is not None and (args.impl != "b200" or args.model == "streaming-0.5b"):
+        ap.error("--dump-outputs writes the outputs of the CUDA frame loop (--impl b200, not --model streaming-0.5b)")
+    return args
+
+
+def dump_outputs(out_dir, arrays):
+    """Write {name: array} as out_dir/<name>.npy in float32.  When the arrays hold more than DUMP_BYTES, every array keeps the same
+    fraction of its elements, at positions drawn from a generator seeded by 0 (sorted, flattened), so that two runs with the same
+    arguments write the same elements.  Their values agree to about 1e-4 rel-L2, not bit for bit: the stream kernel accumulates
+    with fp32 atomics."""
+    arrays = {k: np.ascontiguousarray(v, dtype=np.float32) for k, v in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    budget = DUMP_BYTES - 1024 * len(arrays)                     # room for the .npy headers
+    frac = min(1.0, budget / total) if total else 1.0
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        if frac < 1.0:
+            a = a.reshape(-1)[np.unique(np.random.default_rng(0).integers(0, a.size, int(a.size * frac)))]
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+    log("outputs written to %s: %s%s" % (out_dir, ", ".join("%s %s" % (k, tuple(v.shape)) for k, v in arrays.items()),
+                                           "" if frac == 1.0 else " (seeded %.3f sample of each)" % frac))
 
 
 class ClockSampler:
@@ -239,7 +267,7 @@ def config_dict(args, cfg, L0, F):
 
 # ------------------------------------------------------------------------------------------------------------------
 def run_extra_config(tag, preset, B, L0, F, args, rank, world, local, dev, peak):
-    """Steady-state loop of another BASELINE configuration (same method as `value`): 1 warm-up + 2 timed steps of F frames.
+    """Steady-state loop of another BASELINE configuration (same method as `value`): 1 warm-up + `--steps` timed steps of F frames.
     Every rank executes the same sequence of collectives whether or not its own part failed (a Python-level failure on one rank must
     not leave the others waiting in a barrier): failures are agreed on with a MIN all-reduce after each phase."""
     import torch.distributed as dist
@@ -308,7 +336,7 @@ def run_extra_config(tag, preset, B, L0, F, args, rank, world, local, dev, peak)
     if world > 1:
         dist.barrier()
     torch.cuda.synchronize(dev)
-    K = 2
+    K = args.steps
     ms = 0.0
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     try:
@@ -380,10 +408,14 @@ def run_b200(args):
             model._prefill.run(eng, r, embw[ids[r].to(dev)])
     eng.sync()
     log("weights + prefill(%d tokens) done" % L0)
-    noise_tab = torch.randn(F, B, 64, device=dev)
+    noise_tab = torch.randn(F, B, 64, device=dev, generator=torch.Generator(device=dev).manual_seed(300 + rank))
     ones = [1] * (2 * B)
+    dump = args.dump_outputs is not None and rank == 0
+    if dump:     # per-frame audio and token logits of the last timed step (device-to-device copies on the engine stream)
+        audio_out = torch.empty(F, B, 3200, device=dev)
+        logits_out = torch.empty(F, *eng.logits.shape, device=dev)
 
-    def value_step():
+    def value_step(capture=False):
         eng.codec_state_reset()
         for r in range(B):
             eng.kv_set_len(r, L0); eng.kv_set_len(B + r, 0)
@@ -396,6 +428,10 @@ def run_b200(args):
             with torch.cuda.stream(eng.stream):
                 eng.noise.copy_(noise_tab[f])
             eng.frame_tail(args.cfg_scale)
+            if capture:
+                with torch.cuda.stream(eng.stream):
+                    audio_out[f].copy_(eng.audio)
+                    logits_out[f].copy_(eng.logits)
 
     for _ in range(W):
         value_step()
@@ -406,8 +442,8 @@ def run_b200(args):
     launches0 = eng.launch_count()
     ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     ev0.record(eng.stream)
-    for _ in range(K):
-        value_step()
+    for k in range(K):
+        value_step(capture=dump and k == K - 1)
     ev1.record(eng.stream)
     barrier()
     ms_value = ev0.elapsed_time(ev1)
@@ -540,6 +576,13 @@ def run_b200(args):
 
     # ---------------- BASELINE configs #3 / #4 on the same clock: VibeVoice-7B, short frame counts (the headline stays on config #2) ----
     extra_configs = []
+    if dump:
+        outputs = {"audio": audio_out.permute(1, 0, 2).reshape(B, F * 3200).cpu().numpy(),
+                   "token_logits": logits_out.permute(1, 0, 2).cpu().numpy()}
+        if e2e is not None:
+            outputs["e2e_audio"] = torch.cat(wav).numpy()
+        dump_outputs(args.dump_outputs, outputs)
+
     if args.model == "1.5b" and not args.no_7b:
         model.engine.close()
         del model, eng

@@ -6,6 +6,8 @@ import numpy as np
 import pytest
 import torch
 
+from oracle.make_golden import frame_sample
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
@@ -73,11 +75,10 @@ def test_configs_match_the_shipped_jsons():
         assert sum(math.prod(s) for _, s, _ in param_specs(cfg)) == n_params
     c = preset_config("1.5b")
     assert c.acoustic_tokenizer_config.decoder_depth_list == [8, 3, 3, 3, 3, 3, 3]
-    ref = "/root/reference/vibevoice/configs/qwen2.5_1.5b_64k.json"
-    if os.path.exists(ref):
-        r = VibeVoiceConfig.from_pretrained(ref)
-        assert r.decoder_config.hidden_size == 1536 and r.decoder_config.num_key_value_heads == 2
-        assert r.diffusion_head_config.head_layers == 4 and r.semantic_vae_dim == 128
+    # the 1.5B checkpoint's config.json as published, stored under tests/golden/
+    r = VibeVoiceConfig.from_pretrained(os.path.join(ROOT, "tests", "golden", "qwen2.5_1.5b_64k.json"))
+    assert r.decoder_config.hidden_size == 1536 and r.decoder_config.num_key_value_heads == 2
+    assert r.diffusion_head_config.head_layers == 4 and r.semantic_vae_dim == 128
 
 
 def test_shard_prompts():
@@ -245,6 +246,7 @@ def test_product_generate_host_logic_against_reference_generate_fixture(golden, 
     for r, (a, b) in enumerate(zip(out.speech_outputs, c["audio"])):
         assert (a is None) == (b is None)
         if a is not None:
+            a = frame_sample(a)                                 # the fixture keeps a fixed half of every frame
             assert a.shape == b.shape
             rel = float((a.double() - b.double()).norm() / b.double().norm())
             if case == "quirk" and r == 0:
@@ -287,7 +289,8 @@ def test_product_streaming_and_stop_hooks_against_reference_generate_fixture(gol
                          logits_processor=[ForcedTokenScript(c["scripts"])], **extra)
     assert torch.equal(out.sequences, c["sequences"])
     assert torch.equal(out.reach_max_step_sample, c["reach_max"])
-    for a, b in zip(out.speech_outputs, c["audio"]):
+    for a, b in zip(out.speech_outputs, c["audio"]):                # the fixture keeps a fixed half of every frame
+        a = frame_sample(a)
         assert a.shape == b.shape and float((a.double() - b.double()).norm() / b.double().norm()) < 1e-5
     for r in range(2):
         got = []
@@ -298,6 +301,7 @@ def test_product_streaming_and_stop_hooks_against_reference_generate_fixture(gol
         for x, y in zip(got, want):
             assert (x is None) == (y is None)                      # the stop signal sits where the reference put it
             if x is not None:
+                x = frame_sample(x)
                 assert tuple(x.shape) == tuple(y.shape)
                 assert float((x.double() - y.double()).norm() / y.double().norm()) < 1e-5
 

@@ -5,6 +5,7 @@ import pytest
 import torch
 
 from oracle import vv_oracle as O
+from oracle.make_golden import frame_sample
 from vibevoice_b200.configuration import preset_config
 from vibevoice_b200.synth import synth_state_dict
 
@@ -146,6 +147,7 @@ def test_generate_loop_matches_the_reference_generate(golden, case):
     for a, b in zip(out.speech_outputs, c["audio"]):
         assert (a is None) == (b is None)
         if a is not None:
+            a = frame_sample(a)             # the fixture keeps a fixed half of every frame
             assert a.shape == b.shape
             rel = float((a.double() - b.double()).norm() / b.double().norm())
             assert rel < 1e-5, rel
